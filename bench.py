@@ -9,11 +9,13 @@ rule (image_augmentation.py:21-42), DLA-34-FPN + EMM, fp16 storage / fp32 accumu
 pinned host memory (per frame: H2D, test transform on the device, hot path, packed result D2H -- all inside the wall-clock
 region); `e2e.per_frame_call`: the same frames through model(frame), one blocking call per frame.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype float16|float32]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype float16|float32] [--dump-outputs DIR]
   python bench.py --impl reference ...     # the reference path on the host CPU (oracle port)
   torchrun --nproc-per-node N bench.py --gpus N ...   # one process per GPU, independent streams
 
-Prints ONE JSON line on rank 0.
+Each arm times exactly K steps.  Prints ONE JSON line on rank 0.  --dump-outputs DIR writes what the timed path returned for its
+last step as DIR/<name>.npy (see dump_outputs); the inputs are a pure function of the arguments, so two builds can be compared
+output for output.
 """
 import argparse
 import json
@@ -26,6 +28,7 @@ import time
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True    # the tree may be read-only, and a benchmark run leaves it as it found it
 
 import torch  # noqa: E402
 
@@ -143,12 +146,6 @@ def pin_to_gpu_numa_node(local):
     except Exception:
         pass
     return None
-
-
-def median(xs):
-    xs = sorted(xs)
-    n = len(xs)
-    return xs[n // 2] if n % 2 else 0.5 * (xs[n // 2 - 1] + xs[n // 2])
 
 
 def build_cfg(dtype):
@@ -294,13 +291,28 @@ def kernels_per_frame(h):
     return n
 
 
-REPEATS = 5   # least number of timed regions per arm: the line reports the median region
+SETTLE_S = 0.4   # untimed repeats of an arm's region before its timed one
 
 
-def repeats(steps):
-    """Timed regions per arm: at least REPEATS, and enough short ones to cover ~0.4 s (a 20-step region is 16 ms: one scheduler
-    hiccup on a shared host is 10 % of it, and 5 such regions do not make a stable median; 20 do and still cost < 1 s)."""
-    return REPEATS if REPEATS < 5 else max(REPEATS, min(25, -(-400 // max(int(steps), 1))))
+def settle(run):
+    """Run the arm's K-step region untimed, at least twice and for SETTLE_S: right after set-up the first region runs slow (on a
+    B200 the first of twenty 20-step regions ran at 72 % of the median of the others), and one timed region of K steps must
+    not measure that ramp."""
+    t0, n = time.perf_counter(), 0
+    while n < 2 or time.perf_counter() - t0 < SETTLE_S:
+        run()
+        torch.cuda.synchronize()
+        n += 1
+
+
+def dump_outputs(path, boxes, scores, ids, labels):
+    """What a caller of the timed path receives for its last step, as DIR/<name>.npy: boxes (N x 4, xyxy in network-input
+    pixels) and scores as float32, track ids (-1: a detection no track claimed) and class labels as float64 (exact)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in (("boxes", boxes), ("scores", scores), ("ids", ids), ("labels", labels)):
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64 if a.dtype.kind in "iub" else np.float32))
 
 
 def run_ours(args):
@@ -337,30 +349,26 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     # ---- device-resident arm: `value` (clip API: the detection stage of frame t+1 overlaps the host solver of frame t).
-    # No event timers in this arm (they are on only in the per-frame arm below); REPEATS timed regions of exactly K steps.
+    # No event timers in this arm (they are on only in the per-frame arm below); one timed region of exactly K steps.
     hook = lambda t: h.restore()
-    h.model.forward_clip([frames_dev[i % N_FRAMES] for i in range(max(args.warmup, 4))], before_frame=hook)
-    seq = [frames_dev[(args.warmup + i) % N_FRAMES] for i in range(args.steps)]
     h.eng.timers = None
     sampler = ClockSampler(local)
-    barrier()
     if rank == 0:
         sampler.start()
-    value_ms = []
+    h.model.forward_clip([frames_dev[i % N_FRAMES] for i in range(max(args.warmup, 4))], before_frame=hook)
+    seq = [frames_dev[(args.warmup + i) % N_FRAMES] for i in range(args.steps)]
+    settle(lambda: h.model.forward_clip(seq, before_frame=hook))
+    barrier()
     h.eng.host_timers = {}
-    t_loop0 = time.perf_counter()
-    for rep in range(repeats(args.steps)):
-        barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        results = h.model.forward_clip(seq, before_frame=hook)
-        e1.record()
-        barrier()
-        value_ms.append(e0.elapsed_time(e1))
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    results = h.model.forward_clip(seq, before_frame=hook)
+    e1.record()
+    barrier()
+    ms = e0.elapsed_time(e1)
     host_t, h.eng.host_timers = h.eng.host_timers, None
     ntrk = sum(int((r.get_field("ids") >= 0).sum()) for r in results)
     r = results[-1]
-    ms = median(value_ms)
 
     # ---- end-to-end arm through the public API with HOST frames: `e2e`.  The call a user makes per decoded frame:
     # model(uint8 HWC frame) -> H2D of the frame, test transform on the device, the whole hot path, D2H of the result.
@@ -383,20 +391,18 @@ def run_ours(args):
     def e2e_clip_loop(src):
         h.model.forward_clip([src[i % N_FRAMES] for i in range(max(args.warmup, 4))], before_frame=hook)
         seq_h = [src[(args.warmup + i) % N_FRAMES] for i in range(args.steps)]
-        dts = []
-        for rep in range(repeats(args.steps)):
-            barrier()
-            t0 = time.perf_counter()
-            res = h.model.forward_clip(seq_h, before_frame=hook)
-            torch.cuda.synchronize()
-            dts.append(time.perf_counter() - t0)
-            assert len(res) == args.steps and all(r.bbox.device.type == "cpu" for r in res)
-        return dts, sum(int((r.get_field("ids") >= 0).sum()) for r in res)
+        settle(lambda: h.model.forward_clip(seq_h, before_frame=hook))
+        barrier()
+        t0 = time.perf_counter()
+        res = h.model.forward_clip(seq_h, before_frame=hook)
+        torch.cuda.synchronize()
+        dt = time.perf_counter() - t0
+        assert len(res) == args.steps and all(r.bbox.device.type == "cpu" for r in res)
+        return dt, sum(int((r.get_field("ids") >= 0).sum()) for r in res)
 
-    e2e_clip_s, e2e_clip_err, e2e_clip_all = None, None, []
+    e2e_clip_s, e2e_clip_err = None, None
     try:
-        e2e_clip_all, ntrk_clip = e2e_clip_loop(frames_u8)
-        e2e_clip_s = median(e2e_clip_all)
+        e2e_clip_s, ntrk_clip = e2e_clip_loop(frames_u8)
         if ntrk_clip != ntrk:   # same frames, same restored memory: the from-host clip must track exactly what `value` tracked
             e2e_clip_err = "clip-from-host tracked %d boxes, device-resident clip %d" % (ntrk_clip, ntrk)
     except Exception as exc:   # keep the per-frame number as the headline rather than lose the line
@@ -484,12 +490,11 @@ def run_ours(args):
                          "e2e.per_frame_call: model(frame) once per frame; "
                          "model.results_on_host = True (CPU BoxLists from the packed result block the engine copies D2H)",
                   "baseline_note": "17 FPS = README.md:22 'a single modern GPU', unnamed hardware",
-                  "repeats": "%d timed regions of exactly %d steps per arm; value / e2e are the median region (max over ranks)" % (repeats(args.steps), args.steps),
+                  "timed_steps": "one timed region of exactly %d steps per arm, after untimed repeats of it for >= %.1f s "
+                                 "(max over ranks); e2e may exceed value by a few per cent: the device-resident arm reads 10.8 MB "
+                                 "fp32 frames from HBM (image_to_nhwc), the host arm uploads 2.8 MB uint8 frames and resamples on the "
+                                 "side stream" % (args.steps, SETTLE_S),
                   "numa_cpus_bound": numa_cpus},
-        "spread": {"value_fps": [round(world * args.steps / (x * 1e-3), 1) for x in value_ms],
-                   "e2e_fps": [round(world * args.steps / x, 1) for x in e2e_clip_all],
-                   "note": "this rank's regions; e2e may exceed value by a few per cent: the device-resident arm reads 10.8 MB fp32 "
-                           "frames from HBM (image_to_nhwc), the host arm uploads 2.8 MB uint8 frames and resamples on the side stream"},
         "e2e": {"value": round(e2e_fps, 2), "unit": "frames/s",
                 "api": "model.forward_clip(pinned uint8 host frames)" if clip_ok else "model(pinned uint8 host frame) per frame",
                 "h2d_bytes_per_step": 3 * H_SRC * W_SRC + tp.inputs.numel() * 4,
@@ -523,6 +528,8 @@ def run_ours(args):
                                   "sum + the launch code is the sequential chain of a video"},
         "clocks": clocks,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r.bbox, r.get_field("scores"), r.get_field("ids"), r.get_field("labels"))
     if per_rank is not None:
         out["per_rank_ms"] = {"columns": ["value_region", "per_frame_region", "float_region", "e2e_clip_region", "static_graph", "preprocess"],
                               "rows": per_rank, "gathered_tracks_per_rank": gathered}
@@ -823,14 +830,15 @@ def run_reference(args):
     warm = max(args.warmup, 0)
     for i in range(warm):
         step(i)
-    # bounded: at ~1-2 frames/s the whole run must end within a few minutes
-    steps = min(args.steps, 60)
+    steps = args.steps
     ntrk = 0
     t0 = time.perf_counter()
     for i in range(steps):
         out = step(warm + i)
-        ntrk += int((out["ids"] >= 0).sum()) if isinstance(out, dict) else int((out.get_field("ids") >= 0).sum())
+        ntrk += int((out["ids"] >= 0).sum())
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out["boxes"], out["scores"], out["ids"], out["labels"])
     fps = steps / dt
     world = int(os.environ.get("WORLD_SIZE", 1)) if (args.gpus > 1 and "RANK" in os.environ) else 1
     cfgd = config_dict(world)
@@ -841,7 +849,7 @@ def run_reference(args):
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": cfgd,
         "notes": {"what": "reference algorithm on the host CPU (oracle port, fp32; the reference itself needs maskrcnn_benchmark which "
-                          "is not installable offline); steps capped at 60; rank 0 only, %d torch threads" % cores},
+                          "is not installable offline); rank 0 only, %d torch threads" % cores},
         "cpu_baseline": {"value": round(fps, 4), "unit": "frames/s", "cores": cores, "kind": "port",
                          "sample": "%d full frames (%dx%d, %d tracks) after %d warm-up frames" % (steps, H_NET, W_NET, N_TRACKS, warm)},
         "e2e": {"value": round(fps, 4), "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
@@ -859,6 +867,8 @@ def main():
                     help="information-only A/B arms of the pipeline switches (all of them are measured defaults since round 2, so "
                          "this is off unless asked for): in a child process after the line is final, in this process under a "
                          "watchdog (tests), or not at all (default); 'child' is the child's mode")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's result (boxes, scores, ids, labels) as DIR/<name>.npy")
     ap.add_argument("--workload", default="720p30", choices=sorted(WORKLOADS),
                     help="720p30 = BASELINE.json configs[1] (the metric's configuration, default); 1080p80 = configs[2]; "
                          "r50_720p30 = configs[4]")

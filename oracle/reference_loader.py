@@ -56,6 +56,13 @@ def _patch_color_jitter():
     T.ColorJitter.get_params = staticmethod(get_params)
 
 
+def use_shim():
+    """Put the repository and oracle/shim on sys.path: the stand-ins import without the reference tree."""
+    for p in (_REPO, _SHIM):
+        if p not in sys.path:
+            sys.path.insert(0, p)
+
+
 def load():
     if not available():
         raise RuntimeError("reference tree not present at %s" % REFERENCE_ROOT)

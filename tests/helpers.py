@@ -1,3 +1,5 @@
+import gzip
+import io
 import os
 
 import torch
@@ -31,7 +33,12 @@ def scenario_inputs(name):
 
 
 def load_golden(name):
-    return torch.load(golden_path(name), weights_only=False)
+    """tests/golden/<name>.pt, or <name>.pt.gz where the fixture compresses well."""
+    path = golden_path(name)
+    if not os.path.exists(path):
+        with gzip.open(path + ".gz", "rb") as f:
+            return torch.load(io.BytesIO(f.read()), weights_only=False)
+    return torch.load(path, weights_only=False)
 
 
 def run_oracle_scenario(name):

@@ -39,7 +39,7 @@ def _bench_rank(rank, world, port, q):
     try:
         cabi_emulator.install_for_bench(mpatch)
         import bench
-        mpatch.setattr(bench, "REPEATS", 2)
+        mpatch.setattr(bench, "SETTLE_S", 0.0)
         mpatch.setattr(sys, "argv", ["bench.py", "--gpus", str(world), "--steps", "2", "--warmup", "3", "--dtype", "float32",
                                      "--no-cpu-baseline", "--experimental", "off", "--workload", "selftest"])
         import torch.distributed as dist
@@ -89,7 +89,7 @@ def test_bench_distributed_branch_world2_results_on_host():
     assert len(pr["rows"]) == 2 and len(pr["gathered_tracks_per_rank"]) == 2
     assert all(n > 0 for n in pr["gathered_tracks_per_rank"])        # both ranks' track states arrived
     assert line["e2e"]["clip_error"] is None
-    # value is the whole-job aggregate: 2 ranks x 2 steps over the slowest rank's median region
+    # value is the whole-job aggregate: 2 ranks x 2 steps over the slowest rank's timed region
     assert abs(line["value"] - 2 * 2 / (line["ms_per_step"] * 2 * 1e-3)) / line["value"] < 1e-2
 
 

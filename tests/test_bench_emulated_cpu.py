@@ -12,7 +12,7 @@ import torch
 import cabi_emulator
 
 
-def test_bench_gpu_arm_control_flow_and_json_contract(monkeypatch):
+def test_bench_gpu_arm_control_flow_and_json_contract(monkeypatch, tmp_path):
     cabi_emulator.install_for_bench(monkeypatch)
     import bench
     from siammot_b200 import _lib, ops
@@ -24,7 +24,7 @@ def test_bench_gpu_arm_control_flow_and_json_contract(monkeypatch):
         return out
     monkeypatch.setattr(ops, "xcorr_planar", xcorr_planar_any_dtype)
     monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "2", "--warmup", "3", "--dtype", "float32", "--no-cpu-baseline",
-                                      "--experimental", "inproc", "--workload", "selftest"])
+                                      "--experimental", "inproc", "--workload", "selftest", "--dump-outputs", str(tmp_path / "out")])
     buf = io.StringIO()
     try:
         with contextlib.redirect_stdout(buf):
@@ -44,6 +44,13 @@ def test_bench_gpu_arm_control_flow_and_json_contract(monkeypatch):
     r = line["roofline"]
     assert r["bound"] == "hbm" and r["algorithmic_bytes"] == 8 * 128 * 1381 * 4 and 0 < r["frac"]
     assert line["gpu_launches"] > 0
+    # --dump-outputs: the last timed step's result as float arrays of one box count, tracks in memory among the ids
+    import numpy as np
+    dump = {n: np.load(str(tmp_path / "out" / (n + ".npy"))) for n in ("boxes", "scores", "ids", "labels")}
+    n = dump["boxes"].shape[0]
+    assert dump["boxes"].shape == (n, 4) and n > 0 and all(dump[k].shape == (n,) for k in ("scores", "ids", "labels"))
+    assert dump["boxes"].dtype == dump["scores"].dtype == np.float32 and dump["ids"].dtype == dump["labels"].dtype == np.float64
+    assert int((dump["ids"] >= 0).sum()) >= 4
     # the information-only arms: three-stage clip (K = 2, 3) tracks what the two-stream clip tracks; the planar exchange
     # reproduces the default kernels' windows and responses
     ex = line["experimental"]

@@ -1,21 +1,17 @@
-"""Clip-level result egress (siammot_b200/egress.py) against the reference's own code: ``boxlists_to_entities`` is imported
-verbatim (over stand-ins for gluoncv's two container classes), ``DatasetInference._postprocess_tracks`` is executed from its
-source text (its module needs motmetrics & co. to import).  Needs the reference tree (authoring container)."""
-import ast
-import os
-import sys
-import textwrap
-
-import numpy as np
+"""Clip-level result egress (siammot_b200/egress.py) against the reference's own code: what ``boxlists_to_entities`` (behind the
+per-frame resize / convert of inferencer.py:64-70) and ``DatasetInference._postprocess_tracks`` make of seeded results is stored
+in tests/golden/reference_modules.pt.gz (tests/golden/make_reference_golden.py runs both on the reference)."""
 import pytest
 import torch
 
-from oracle import reference_loader
+from helpers import load_golden
 
-pytestmark = pytest.mark.skipif(not reference_loader.available(), reason="reference tree not present")
+CLASSES = ("person", "vehicle")
+VIDEOS = [(1280, 720), (1920, 1080), (2560, 1408)]
+POSTPROCESS = dict(seed=7, frames=40, track_len=5, track_conf=0.7)
 
 
-def _random_results(seed, n_frames=12, net=(1280, 704)):
+def random_results(seed, n_frames=12, net=(1280, 704)):
     from siammot_b200.structures import BoxList
     g = torch.Generator().manual_seed(seed)
     out = []
@@ -31,60 +27,26 @@ def _random_results(seed, n_frames=12, net=(1280, 704)):
     return out
 
 
-@pytest.mark.parametrize("video", [(1280, 720), (1920, 1080), (2560, 1408)])
+@pytest.mark.parametrize("video", VIDEOS)
 def test_clip_to_tracks_and_entities_equal_the_reference_path(video):
-    reference_loader.load()
-    from maskrcnn_benchmark.structures.bounding_box import BoxList as RefBoxList
-    from siammot.utils.boxlists_to_entities import boxlists_to_entities
     from siammot_b200 import egress
-    results = _random_results(video[0])
-    # the reference path, per frame (inferencer.py:64-70)
-    ref_entities = []
-    for t, r in enumerate(results):
-        rb = RefBoxList(r.bbox.clone(), r.size, "xyxy")
-        for f in r.fields():
-            rb.add_field(f, r.get_field(f))
-        o = rb.resize([video[0], video[1]]).convert("xywh").to(torch.device("cpu"))
-        ref_entities += boxlists_to_entities([o], 100 + t, [0.04 * (100 + t)], class_table=["person", "vehicle"])
+    ref_entities = load_golden("reference_modules")["egress"][video]
+    results = random_results(video[0])
     tracks = egress.clip_to_tracks(results, video[0], video[1], first_frame_idx=100, timestamps=[0.04 * (100 + t) for t in range(len(results))])
-    got = egress.to_entities(tracks, class_table=["person", "vehicle"])
+    got = egress.to_entities(tracks, class_table=list(CLASSES))
     assert len(got) == len(ref_entities) == len(tracks)
     for a, b in zip(got, ref_entities):
-        assert a.bbox == b.bbox and a.confidence == b.confidence and a.labels == b.labels
-        assert a.id == b.id and a.frame_num == b.frame_num and a.time == b.time
-
-
-def _reference_postprocess():
-    """DatasetInference._postprocess_tracks, literally, from the reference file."""
-    path = os.path.join(reference_loader.REFERENCE_ROOT, "siammot", "engine", "inferencer.py")
-    src = open(path).read()
-    tree = ast.parse(src)
-    for node in ast.walk(tree):
-        if isinstance(node, ast.FunctionDef) and node.name == "_postprocess_tracks":
-            code = textwrap.dedent(ast.get_source_segment(src, node))
-            break
-    else:
-        raise AssertionError("_postprocess_tracks not found")
-    from gluoncv.torch.data.gluoncv_motion_dataset.dataset import DataSample
-    ns = {"np": np, "DataSample": DataSample}
-    exec(code, ns)
-    return ns["_postprocess_tracks"], DataSample
+        assert a.bbox == b["bbox"] and a.confidence == b["confidence"] and a.labels == b["labels"]
+        assert a.id == b["id"] and a.frame_num == b["frame_num"] and a.time == b["time"]
 
 
 def test_postprocess_tracks_equals_the_reference_filter():
-    reference_loader.load()
     from siammot_b200 import egress
-    fn, DataSample = _reference_postprocess()
-
-    class Self(object):
-        _track_len, _track_conf = 5, 0.7
-    results = _random_results(7, n_frames=40)
-    tracks = egress.clip_to_tracks(results, 1280, 720)
-    sample = DataSample("v", entities=egress.to_entities(tracks, ["person", "vehicle"]))
-    ref = fn(Self(), sample).entities
-    got = egress.to_entities(egress.postprocess_tracks(tracks, 5, 0.7), ["person", "vehicle"])
+    ref = load_golden("reference_modules")["postprocess"]
+    tracks = egress.clip_to_tracks(random_results(POSTPROCESS["seed"], n_frames=POSTPROCESS["frames"]), 1280, 720)
+    got = egress.to_entities(egress.postprocess_tracks(tracks, POSTPROCESS["track_len"], POSTPROCESS["track_conf"]), list(CLASSES))
     key = lambda e: (e.id, e.frame_num, tuple(e.bbox))
-    assert len(ref) > 0 and sorted(map(key, ref)) == sorted(map(key, got))
+    assert len(ref) > 0 and ref == sorted(map(key, got))
     assert all(e.id >= 0 for e in got)
     # grouped by id, frames ascending
     assert [(e.id, e.frame_num) for e in got] == sorted((e.id, e.frame_num) for e in got)

@@ -194,44 +194,33 @@ def test_search_region_numpy_twin_is_bit_exact():
         assert np.array_equal(tu.search_region_np(boxes.numpy()), ref.numpy())
 
 
-@pytest.mark.parametrize("name", ["emm_256x384", "emm_r50_192x320", "emm_dla102_192x320", "emm_dla60_dcn_192x320"])
-def test_state_dict_layout_equals_the_reference_module_tree(name):
-    """build_siammot(cfg).state_dict() has exactly the keys and shapes of the reference's SiamMOT (DLA-34-FPN and the upstream
-    R-50-FPN body), so DetectronCheckpointer-style checkpoints load unchanged.  Needs the reference tree (authoring container)."""
+LAYOUT_SCENARIOS = ["emm_256x384", "emm_r50_192x320", "emm_dla102_192x320", "emm_dla60_dcn_192x320"]
+
+
+def _reference_layout(name):
+    """The keys and shapes of the reference's SiamMOT state dict (tests/golden/make_reference_golden.py)."""
     import sys
     sys.path.insert(0, os.path.join(REPO, "tests"))
-    from oracle import reference_loader
-    if not reference_loader.available():
-        pytest.skip("reference tree not present")
+    from helpers import load_golden
+    return dict(load_golden("reference_modules")["layout"][name])
+
+
+@pytest.mark.parametrize("name", LAYOUT_SCENARIOS)
+def test_state_dict_layout_equals_the_reference_module_tree(name):
+    """build_siammot(cfg).state_dict() has exactly the keys and shapes of the reference's SiamMOT (DLA-34-FPN and the upstream
+    R-50-FPN body), so DetectronCheckpointer-style checkpoints load unchanged."""
     from helpers import scenario_cfg
-    from scenarios import ORACLE_SCENARIOS, SCENARIOS
     from siammot_b200.modelling import build_siammot
-    sc = SCENARIOS.get(name) or ORACLE_SCENARIOS[name]
-    cfg0, build = reference_loader.load()
-    rcfg = cfg0.clone()
-    rcfg.merge_from_file(os.path.join(reference_loader.REFERENCE_ROOT, "configs", "dla", sc["yaml"]))
-    rcfg.merge_from_list(sc["overrides"])
-    rcfg.MODEL.DEVICE = "cpu"
-    ref = {k: tuple(v.shape) for k, v in build(rcfg).state_dict().items()}
+    ref = _reference_layout(name)
     ours = {k: tuple(v.shape) for k, v in build_siammot(scenario_cfg(name)).state_dict().items()}
     assert ours == ref
 
 
 def test_detector_only_state_dict_layout_equals_the_reference():
     """MODEL.TRACK_ON False: no roi_heads.track.* parameters on either side (roi_heads.py:87-100)."""
-    import sys
-    sys.path.insert(0, os.path.join(REPO, "tests"))
-    from oracle import reference_loader
-    if not reference_loader.available():
-        pytest.skip("reference tree not present")
+    ref = _reference_layout("detector_only")
     from helpers import scenario_cfg
     from siammot_b200.modelling import build_siammot
-    cfg0, build = reference_loader.load()
-    rcfg = cfg0.clone()
-    rcfg.merge_from_file(os.path.join(reference_loader.REFERENCE_ROOT, "configs", "dla", "DLA_34_FPN_EMM.yaml"))
-    rcfg.merge_from_list(["MODEL.TRACK_ON", False])
-    rcfg.MODEL.DEVICE = "cpu"
-    ref = {k: tuple(v.shape) for k, v in build(rcfg).state_dict().items()}
     cfg = scenario_cfg("emm_256x384")
     cfg.merge_from_list(["MODEL.TRACK_ON", False])
     ours = {k: tuple(v.shape) for k, v in build_siammot(cfg).state_dict().items()}

@@ -59,17 +59,19 @@ def test_golden_scenarios_exercise_the_state_machine():
     assert expired, "no track expired"
 
 
-@pytest.mark.skipif(not __import__("oracle.reference_loader", fromlist=["x"]).available(),
-                    reason="reference tree not present (authoring container only)")
-def test_oracle_matches_live_reference_xcorr():
-    """xcorr.py imports verbatim (pure torch): compare the restatement with it directly."""
-    from oracle import reference_loader
-    reference_loader.load()
-    from siammot.modelling.track_head.EMM.xcorr import xcorr_depthwise as ref_xcorr
-    from oracle.siammot_oracle import xcorr_depthwise
+def xcorr_inputs():
     torch.manual_seed(0)
-    x, k = torch.randn(5, 16, 30, 30), torch.randn(5, 16, 15, 15)
-    assert torch.equal(ref_xcorr(x, k), xcorr_depthwise(x, k))
+    return torch.randn(5, 16, 30, 30), torch.randn(5, 16, 15, 15)
+
+
+def test_oracle_matches_reference_xcorr():
+    """The restatement of xcorr.py (pure torch) against the reference's own output on the same inputs
+    (tests/golden/make_reference_golden.py stores a fixed sample of it)."""
+    from oracle.siammot_oracle import xcorr_depthwise
+    gold = load_golden("reference_modules")["xcorr"]
+    got = xcorr_depthwise(*xcorr_inputs())
+    assert tuple(got.shape) == gold["shape"]
+    assert torch.equal(got.reshape(-1)[gold["idx"].long()], gold["val"])
 
 
 def test_oracle_matches_reference_golden_with_given_detections():

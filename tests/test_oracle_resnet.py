@@ -64,11 +64,9 @@ def test_oracle_resnet50_matches_torchvision_with_strides_on_the_1x1():
 def test_shim_resnet50_matches_oracle():
     """The nn.Module restatement the golden generator runs the reference on == the functional restatement that travels."""
     from oracle import reference_loader
-    if not reference_loader.available():
-        pytest.skip("reference tree not present (GPU box)")
     from oracle import siammot_oracle as orc
     cfg, sd, clip = _cfg_and_weights()
-    reference_loader.load()
+    reference_loader.use_shim()
     from maskrcnn_benchmark.config import cfg as ucfg
     from maskrcnn_benchmark.modeling.backbone import resnet
     c = ucfg.clone()
